@@ -21,7 +21,8 @@ Order of a run (engine arm):
      strong_256 (N > 1: 256 utterances TOTAL, LPT-sharded over the ranks), mtl_256 (config 4, multilingual vocabulary,
      256 total), turbo_512 (config 5, Turbo 350M, 512 total, 2-step meanflow), b1_latency (config 2);
   5. `cpu_baseline` (rank 0, N = 1 only): k = 4 utterances of the batch (sorted indices 0 / 85 / 170 / 255) through the
-     reference's CPU path (the unmodified reference when /root/reference is importable, else the oracle port).
+     reference's CPU path (the oracle port of the reference algorithm).
+  --dump-outputs DIR: after the timed steps, the waveforms of the last one (see dump_outputs) for output comparison.
 """
 import argparse
 import json
@@ -126,36 +127,22 @@ def cpu_model():
 # ------------------------------------------------------------------------------------------------ CPU reference arm
 class CpuReference:
     """The reference's CPU path for one utterance at a time (the reference is batch-1): T3.inference (CFG pair, sampler
-    defaults of generate(): T 0.8, min_p 0.05, rep 1.2, cfg 0.5) -> token clean-up -> flow (10 NFE) -> HiFT.
-    kind = 'reference': the UNMODIFIED reference modules imported from /root/reference (authoring container only);
-    kind = 'port': the oracle restatement of the same algorithm (the GPU box has no /root/reference)."""
+    defaults of generate(): T 0.8, min_p 0.05, rep 1.2, cfg 0.5) -> token clean-up -> flow (10 NFE) -> HiFT, run by the
+    oracle restatement of the same algorithm (kind = 'port')."""
 
     def __init__(self, threads=None):
         from oracle import weights as W
+        from oracle.t3_ref import T3Oracle
+        from oracle.flow_ref import FlowOracle
+        from oracle.hift_ref import HiFTOracle
         self.threads = threads or host_threads()
         torch.set_num_threads(self.threads)
         self.W = W
         self.c3, self.cg = W.make_conds(1234)
         self.kind = "port"
-        if os.path.isdir("/root/reference/src/chatterbox") and os.environ.get("CBX_CPU_ARM", "auto") != "port":
-            try:
-                from oracle import ref_harness as R
-                R.install()
-                from chatterbox.models.t3.modules.cond_enc import T3Cond
-                self.t3 = R.build_t3(); self.t3.load_state_dict(W.make_t3_weights(0), strict=True)
-                self.flow = R.build_flow(); self.flow.load_state_dict(W.make_flow_weights(0), strict=True)
-                self.hift = R.build_hift(); self.hift.load_state_dict(W.make_hift_weights(0), strict=True)
-                self.T3Cond = T3Cond
-                self.kind = "reference"
-            except Exception as e:          # pragma: no cover - depends on the container
-                log(f"reference import failed ({e!r}); using the oracle port")
-        if self.kind == "port":
-            from oracle.t3_ref import T3Oracle
-            from oracle.flow_ref import FlowOracle
-            from oracle.hift_ref import HiFTOracle
-            self.t3 = T3Oracle(W.make_t3_weights(0))
-            self.flow = FlowOracle(W.make_flow_weights(0))
-            self.hift = HiFTOracle(W.make_hift_weights(0))
+        self.t3 = T3Oracle(W.make_t3_weights(0))
+        self.flow = FlowOracle(W.make_flow_weights(0))
+        self.hift = HiFTOracle(W.make_hift_weights(0))
 
     def utterance(self, text, budget, seed=0):
         """-> (audio_seconds, wall_seconds, split)"""
@@ -163,34 +150,17 @@ class CpuReference:
         tt = torch.stack([tt, tt])
         torch.manual_seed(seed)
         t0 = time.perf_counter()
-        if self.kind == "reference":
-            c3 = self.c3
-            cond = self.T3Cond(speaker_emb=c3["speaker_emb"], cond_prompt_speech_tokens=c3["cond_prompt_speech_tokens"],
-                               emotion_adv=c3["emotion_adv"])
-            with torch.inference_mode():
-                toks = self.t3.inference(t3_cond=cond, text_tokens=tt, max_new_tokens=int(budget), temperature=0.8, top_p=1.0,
-                                         min_p=0.05, repetition_penalty=1.2, cfg_weight=0.5)
-        else:
-            toks = self.t3.inference(self.c3, tt, int(budget), temperature=0.8, top_p=1.0, min_p=0.05, repetition_penalty=1.2,
-                                     cfg_weight=0.5)
+        toks = self.t3.inference(self.c3, tt, int(budget), temperature=0.8, top_p=1.0, min_p=0.05, repetition_penalty=1.2,
+                                 cfg_weight=0.5)
         t1 = time.perf_counter()
         sp = toks[0]
         eos = (sp == 6562).nonzero()
         if len(eos):
             sp = sp[:int(eos[0])]
         sp = sp[sp < 6561]
-        if self.kind == "reference":
-            cg = self.cg
-            with torch.inference_mode():
-                mel, _ = self.flow.inference(token=sp[None], token_len=torch.tensor([sp.numel()]), prompt_token=cg["prompt_token"],
-                                             prompt_token_len=cg["prompt_token_len"], prompt_feat=cg["prompt_feat"],
-                                             prompt_feat_len=None, embedding=cg["embedding"], finalize=True, n_timesteps=10)
-                t2 = time.perf_counter()
-                self.hift.inference(speech_feat=mel)
-        else:
-            mel = self.flow.inference(sp, self.cg, 10)
-            t2 = time.perf_counter()
-            self.hift.inference(mel)
+        mel = self.flow.inference(sp, self.cg, 10)
+        t2 = time.perf_counter()
+        self.hift.inference(mel)
         t3 = time.perf_counter()
         return sp.numel() / 25.0, t3 - t0, dict(t3_s=round(t1 - t0, 2), flow_s=round(t2 - t1, 2), hift_s=round(t3 - t2, 2),
                                                 tokens=int(sp.numel()), n_text=int(text.numel()))
@@ -236,9 +206,8 @@ def run_reference(args, rank, world):
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": 1000.0 * wall / args.steps, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic", "rtf": wall / audio,
-            "config": {"workload": WORKLOAD, "arm": ("the unmodified reference modules on CPU" if ref.kind == "reference" else
-                                                      "CPU oracle port of the reference algorithm (fp32, torch CPU ops in the reference's order)")
-                       + ", bounded sample of the workload: one utterance per step",
+            "config": {"workload": WORKLOAD, "arm": "CPU oracle port of the reference algorithm (fp32, torch CPU ops in the reference's "
+                                                    "order), bounded sample of the workload: one utterance per step",
                        "sample": sample, "split_s": split, "cpu_model": cpu_model()},
             "cpu_baseline": {"value": v, "unit": UNIT, "cores": ref.threads, "kind": ref.kind, "sample": sample},
             "e2e": {"value": v, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
@@ -259,6 +228,26 @@ def stage_work(texts, lens, n_layers=30, cfg_rows=2, nfe=10, prompt=N_PROMPT):
     flow_flops = float((113.2e6 * nn + 90.1e3 * nn * nn).sum()) + nfe * cfg_rows * float((T * (132161536.0 + 114688.0 * T)).sum())
     frames = float((2.0 * n).sum())
     return dict(t3_bytes=t3_bytes, flow_flops=flow_flops, hift_flops=612.3e6 * frames, hift_bytes=0.30e6 * frames, frames=frames)
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_sample(n_utts, budget_max):
+    """Utterances whose whole waveforms --dump-outputs writes: a fixed, seeded subset, as many as fit in DUMP_BYTES at the
+    longest possible waveform (960 float32 samples per speech token), less 1 MB for the lengths and the file headers."""
+    k = max(1, min(n_utts, (DUMP_BYTES - 1_000_000) // (960 * 4 * budget_max)))
+    return sorted(torch.randperm(n_utts, generator=torch.Generator().manual_seed(SEED))[:k].tolist())
+
+
+def dump_outputs(out_dir, wavs, budget_max):
+    """What generate_batch returned in the last timed step: wav_lengths.npy (float64 [B], samples of every waveform) and
+    wav_<b>.npy (float32) for the utterances of dump_sample()."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "wav_lengths.npy"), np.array([w.numel() for w in wavs], dtype=np.float64))
+    for b in dump_sample(len(wavs), budget_max):
+        np.save(os.path.join(out_dir, f"wav_{b:03d}.npy"), wavs[b].detach().float().cpu().numpy())
+    log(f"wrote the last timed step's outputs to {out_dir}")
 
 
 # ------------------------------------------------------------------------------------------------ this engine
@@ -317,6 +306,8 @@ def run_engine(args, rank, world, local_rank):
     log(f"models loaded; batch={args.batch} sum_budget={sum(budgets)}")
 
     def one_pass(to_host, tm, tx=texts, bd=budgets, model=None):
+        # the CFM start noise is drawn from torch's global generator, which torch seeds at random in every process
+        torch.manual_seed(SEED + rank)
         return (model or tts).generate_batch(tx, max_new_tokens=bd, seed=1000 * rank, kv_dtype="bf16", to_host=to_host, timings=tm)
 
     # ---- 1. warm-up + timed region (device-resident inputs, no kernel timers)
@@ -329,8 +320,18 @@ def run_engine(args, rank, world, local_rank):
     clocks = ClockSampler(local_rank)
     if rank == 0:
         clocks.start()
-    ms, wall, tms = timed(lambda tm: one_pass(False, tm), args.steps)
+    last = {"n": 0}
+
+    def timed_step(tm):
+        wavs = one_pass(False, tm)
+        last["n"] += 1
+        if last["n"] == args.steps:       # only the last step's waveforms outlive their step
+            last["wavs"] = wavs
+
+    ms, wall, tms = timed(timed_step, args.steps)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last.pop("wavs"), args.budget_max)
     launches = eng.h.launch_count() - launches0
     stats_timed = dict(eng.stats)
     audio_total = allsum(sum(t["audio_s"] for t in tms))
@@ -557,7 +558,10 @@ def main():
     ap.add_argument("--no-profile", action="store_true", help="skip the per-kernel-class profiling passes")
     ap.add_argument("--no-extra", action="store_true", help="skip strong scaling / multilingual / Turbo / B=1 passes")
     ap.add_argument("--cpu-sample", default="k4", choices=["k4", "none"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the waveforms of the last timed step (rank 0) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))

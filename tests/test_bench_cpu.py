@@ -41,6 +41,24 @@ def test_stage_work_model_matches_the_baseline_formulas():
     assert np.isclose(w["hift_flops"], 612.3e6 * 1000) and np.isclose(w["hift_bytes"], 0.30e6 * 1000)
 
 
+def test_dump_outputs_sample_is_fixed_and_bounded(tmp_path):
+    """--dump-outputs: the same utterances every run, whole waveforms within 64 MB even when every utterance reaches its
+    budget, float32 waveforms + float64 lengths of the whole batch."""
+    b = _bench()
+    for budget_max in (1000, 75, 20000):
+        idx = b.dump_sample(256, budget_max)
+        assert idx == b.dump_sample(256, budget_max) and idx == sorted(set(idx)) and 0 <= idx[0] and idx[-1] < 256
+        assert len(idx) == 1 or len(idx) * budget_max * 960 * 4 + 256 * 8 <= b.DUMP_BYTES
+    assert len(b.dump_sample(256, 1000)) == 16 and b.dump_sample(3, 10) == [0, 1, 2]
+    wavs = [torch.full((960 * n,), float(n)) for n in (5, 0, 7, 3)]
+    b.dump_outputs(str(tmp_path), wavs, 10)
+    assert np.load(tmp_path / "wav_lengths.npy").tolist() == [4800.0, 0.0, 6720.0, 2880.0]
+    for i in b.dump_sample(4, 10):
+        w = np.load(tmp_path / f"wav_{i:03d}.npy")
+        assert w.dtype == np.float32 and np.array_equal(w, wavs[i].numpy())
+    assert sum(f.stat().st_size for f in tmp_path.iterdir()) <= b.DUMP_BYTES
+
+
 def test_tool_scripts_compile():
     for f in glob.glob(os.path.join(ROOT, "tools", "*.py")) + [os.path.join(ROOT, "bench.py"), os.path.join(ROOT, "__graft_entry__.py")]:
         py_compile.compile(f, doraise=True)
